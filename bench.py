@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--metric sort|reduce]      (N > 1: launched by torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W [--metric sort|reduce]
+  python bench.py ... --dump-outputs DIR      (also writes what the last timed step computed, see write_outputs)
 
 One "step" = one pass of the hot path over one synthetic batch (SURVEY.md §8d generators, seed 42):
   sort   : DIA<uint64_t>::Sort of 1e8 uniform keys per GPU          (BASELINE.json configs[1]; weak scaling)
@@ -38,6 +39,7 @@ SORT_PASS_BYTES_PER_KEY = 16.0          # one stable partition pass: read 8 + wr
 SORT_MODEL_BYTES_PER_KEY = {1: 136.0}   # SURVEY.md §8(d): LSB radix sort, p = 1; p > 1: 184
 REDUCE_PASS_BYTES_PER_RECORD = 32.0     # one hash-digit partition pass: read 16 + write 16
 REDUCE_MODEL_BYTES_PER_RECORD = 25.5    # SURVEY.md §8(d): 16 B/record + 64 B x D_local/N_local for Zipf(1, 2^26), 1.25e8 per GPU
+DUMP_ITEMS = 1 << 20                    # --dump-outputs: items written per job (at most 4 float64 arrays of them: 32 MiB)
 
 
 def measured_peaks():
@@ -228,7 +230,8 @@ def main_reference(args):
         if metric != "sort":
             print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/thrill_ref_driver is not built and the C port has no timed reduce leg"}))
             return 0
-        t = run_oracle_port_sort(n // 10)
+        times = [run_oracle_port_sort(n // 10) for _ in range(args.warmup + args.steps)][args.warmup:]
+        t = sum(times) / len(times)
         value, cores, kind, sample = (n // 10) / t, 1, "port", "oracle C port on %d keys" % (n // 10)
         ms = t * 1e3
     else:
@@ -274,9 +277,31 @@ def zipf_cdf_numpy(universe, s=1.0):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step handed to its caller, so that two builds can be compared output for output
 
-def bench_sort(args, ctx, world, rank, hbm_peak, peak_src, zipf=False, d_cdf=None, steps=None, warmup=None, e2e=True):
-    """device-resident Sort of n u64 keys per GPU (+ the end-to-end form); returns the line's fields"""
+def write_outputs(out_dir, prefix, world, rank, keys, vals=None):
+    """Writes <prefix>_count (items this rank received) and, at fixed positions of the output in key order, <prefix>_index,
+    the u64 keys split into exact halves <prefix>_keys_hi32 / _lo32 and, for a reduce, the f64 sums <prefix>_vals; all
+    float64 .npy.  Outputs of more than DUMP_ITEMS / world items are sampled at positions drawn with the fixed seed, so equal
+    outputs give equal files.  Ranks of a multi-GPU job write <name>_rank<r>.npy."""
+    n = len(keys)
+    take = DUMP_ITEMS // world
+    idx = np.arange(n) if n <= take else np.sort(np.random.default_rng(SEED).choice(n, take, replace=False))
+    k = keys[idx]
+    arrays = {"count": [n], "index": idx, "keys_hi32": k >> np.uint64(32), "keys_lo32": k & np.uint64(0xFFFFFFFF)}
+    if vals is not None:
+        arrays["vals"] = vals[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else "_rank%d" % rank
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, "%s_%s%s.npy" % (prefix, name, suffix)), np.asarray(a, dtype=np.float64))
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+
+def bench_sort(args, ctx, world, rank, hbm_peak, peak_src, zipf=False, d_cdf=None, steps=None, warmup=None, e2e=True, dump=None):
+    """device-resident Sort of n u64 keys per GPU (+ the end-to-end form); returns the line's fields.  dump: directory for
+    write_outputs of the last timed step"""
     from thrill_b200 import api, capi
     tg = ctx.tg
     L = tg.L
@@ -337,6 +362,8 @@ def bench_sort(args, ctx, world, rank, hbm_peak, peak_src, zipf=False, d_cdf=Non
                         and parity["multiset_xor_match"] and ordered and balance <= 1.5)
     if not parity["ok"]:
         raise SystemExit("bench: sort parity check FAILED: %s" % json.dumps(parity))
+    if dump:
+        write_outputs(dump, "sort", world, rank, tg.download(out_p.value, out_n.value * 8, np.uint64))
 
     ms_per_step = sum(step_ms) / len(step_ms)
     value = n * world / (ms_per_step / 1e3)
@@ -458,10 +485,10 @@ def bench_terasort(args, ctx, world, rank, hbm_peak, steps=2, warmup=1):
 
 
 def e2e_in_thrill(n=20000000):
-    """The drop-in inside a real Thrill job (tests/host/gpu_nodes_test: api::Run, 1 worker, the unmodified reference library
-    around the GPU nodes): wall time of Generate -> thrill_gpu::Sort -> AllGather against the stock Sort on the same worker
+    """The drop-in inside a real Thrill job (tests/host/gpu_nodes_test.cpp, built into oracle/_ref/host: api::Run, 1 worker,
+    the unmodified reference library around the GPU nodes): wall time of Generate -> thrill_gpu::Sort -> AllGather against the stock Sort on the same worker
     thread.  BlockPool memory is pageable here: this is the number a Thrill user gets without pinning it."""
-    exe = os.path.join(ROOT, "tests", "host", "_build", "gpu_nodes_test")
+    exe = os.path.join(ROOT, "oracle", "_ref", "host", "gpu_nodes_test")
     if not os.path.exists(exe):
         return None
     env = dict(os.environ, THRILL_NET="mock", THRILL_LOCAL="1", THRILL_WORKERS_PER_HOST="1", THRILL_LOG="")
@@ -469,7 +496,7 @@ def e2e_in_thrill(n=20000000):
         res = subprocess.run([exe, str(n)], env=env, capture_output=True, text=True, timeout=600)
     except Exception as e:          # noqa: BLE001
         return {"error": str(e)[:200]}
-    out = {"binary": "tests/host/_build/gpu_nodes_test %d (THRILL_WORKERS_PER_HOST=1)" % n, "rc": res.returncode, "sections": []}
+    out = {"binary": "oracle/_ref/host/gpu_nodes_test %d (THRILL_WORKERS_PER_HOST=1)" % n, "rc": res.returncode, "sections": []}
     for l in res.stdout.splitlines():
         if l.startswith(("PASS", "FAIL")):
             out["sections"].append(l[:160])
@@ -503,7 +530,9 @@ def reduce_parity(ctx, world, rank, d_cdf):
             "every_key_on_hash_owner": all(p[2] for p in parts)}
 
 
-def bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf, steps=None, warmup=None, e2e=True, uniform=False):
+def bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf, steps=None, warmup=None, e2e=True, uniform=False, dump=None):
+    """device-resident ReducePair of rn records per GPU (+ the end-to-end form); returns the line's fields.  dump: directory
+    for write_outputs of the last timed step"""
     from thrill_b200 import api, capi
     tg = ctx.tg
     L = tg.L
@@ -543,6 +572,11 @@ def bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf, steps=None, 
                                                         ("segcount", capi.K_SEGCOUNT), ("exchange", capi.K_EXCHANGE),
                                                         ("preagg", capi.K_PREAGG))}
     tg.profile_enable(False)
+    if dump:        # before the parity sample below, whose operator call reuses the output buffer
+        out = tg.download(rp.value, rcount.value * 16, np.dtype([("key", "<u8"), ("val", "<f8")]))
+        out = out[np.argsort(out["key"], kind="stable")]          # the operator's output order is unspecified
+        write_outputs(dump, "reduce", world, rank, out["key"], out["val"])
+        del out
     # parity of the measured run: ownership of (a sample of) the output keys, then the exact-mode sample
     nchk = min(int(rcount.value), 1 << 20)
     okeys = tg.download(rp.value, nchk * 16, np.dtype([("key", "<u8"), ("val", "<f8")]))["key"] if nchk else np.zeros(0, np.uint64)
@@ -627,8 +661,13 @@ def main():
     ap.add_argument("--terasort-n", type=int, default=125000000, help="TeraSort records per GPU of the extra (0 = skip)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="only the metric itself (no second operator, no Zipf sort)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the metric's last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU arm's outputs; --impl reference has none to write")
         return main_reference(args)
 
     from thrill_b200 import api
@@ -644,7 +683,7 @@ def main():
     d_cdf = tg.to_device(zipf_cdf_numpy(ZIPF_UNIVERSE))
     extra = {}
     if args.metric == "sort":
-        main_res = bench_sort(args, ctx, world, rank, hbm_peak, peak_src)
+        main_res = bench_sort(args, ctx, world, rank, hbm_peak, peak_src, dump=args.dump_outputs)
         if not args.no_extras:
             try:        # an extra must never cost the headline line
                 z = bench_sort(args, ctx, world, rank, hbm_peak, peak_src, zipf=True, d_cdf=d_cdf, steps=3, warmup=2, e2e=False)
@@ -667,7 +706,7 @@ def main():
                     extra["terasort"] = {"error": str(e)[:300]}
         name, unit, dtype, n_item = "sort_keys_per_s", "keys/s", "u64", args.n
     else:
-        main_res = bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf)
+        main_res = bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf, dump=args.dump_outputs)
         if not args.no_extras:
             try:
                 u = bench_reduce(args, ctx, world, rank, hbm_peak, peak_src, d_cdf, steps=3, warmup=2, e2e=False, uniform=True)

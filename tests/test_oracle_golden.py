@@ -1,15 +1,16 @@
 """Pins oracle/thrill_oracle.c against outputs of the UNMODIFIED reference:
 (1) the committed fixtures tests/golden/reference_outputs.npz (made by tests/golden/make_golden.py),
-(2) when the prebuilt reference binary is present (oracle/_ref/thrill_ref_driver), live runs on fresh inputs.
+(2) tests/golden/reference_outputs_live.npz (made by tests/golden/make_golden_live.py), the reference's runs on file
+inputs and fresh shapes.
 CPU only."""
 import os
-import tempfile
 
 import numpy as np
 import pytest
 
 import oracle_lib as O
-from golden_util import REDUCE_OUT, golden, golden_r2, sha
+from golden_util import (LIVE_REDUCE_TO_INDEX_CASES, LIVE_REDUCE_ZERO_KEY_WORKERS, LIVE_SORT_CASES, golden, golden_live,
+                         golden_r2, live_reduce_zero_key_input, live_sort_input, sha)
 
 
 def _counts(n, p):
@@ -81,40 +82,19 @@ def test_golden_terasort_records():
     assert sha(out) == str(g["terasort_20000_w3_sha256"])
 
 
-# ---- live runs of the reference itself (binary prebuilt in oracle/_ref; skipped if absent) ----
-needs_ref = pytest.mark.skipif(not O.have_ref_driver(), reason="oracle/_ref/thrill_ref_driver not built")
-
-
-@needs_ref
-@pytest.mark.ref
-@pytest.mark.parametrize("workers,n", [(1, 30000), (2, 1), (3, 12345), (8, 200000)])
+# ---- the reference's runs on file inputs and fresh shapes (outputs stored by tests/golden/make_golden_live.py) ----
+@pytest.mark.parametrize("workers,n", LIVE_SORT_CASES)
 def test_live_reference_sort_file_input(workers, n):
-    rng = np.random.RandomState(workers * 1000 + n % 997)
-    keys = rng.randint(0, 50, size=n).astype(np.uint64) if workers == 3 else \
-        rng.randint(0, 2**63, size=n).astype(np.uint64)
-    with tempfile.TemporaryDirectory() as d:
-        keys.tofile(os.path.join(d, "in.bin"))
-        O.run_ref_driver(workers=workers, op="sort_u64", gen="file", out=os.path.join(d, "o.bin"),
-                         **{"in": os.path.join(d, "in.bin")})
-        ref = np.fromfile(os.path.join(d, "o.bin"), dtype=np.uint64)
+    keys = live_sort_input(workers, n)
     out, _ = O.sort_operator(keys, _counts(n, workers))
-    assert np.array_equal(out.view(np.uint64), ref)
+    assert sha(out.view(np.uint64)) == str(golden_live()["sort_file_w%d_n%d_sha256" % (workers, n)])
 
 
-@needs_ref
-@pytest.mark.ref
-@pytest.mark.parametrize("workers", [1, 2, 5])
+@pytest.mark.parametrize("workers", LIVE_REDUCE_ZERO_KEY_WORKERS)
 def test_live_reference_reduce_with_zero_key(workers):
-    rng = np.random.RandomState(workers)
-    n = 60000
-    kv = np.zeros(n, dtype=O.KV)
-    kv["key"] = rng.randint(0, 500, size=n)          # includes key 0: sentinel slot path
-    kv["val"] = rng.randint(0, 1000, size=n)
-    with tempfile.TemporaryDirectory() as d:
-        kv.tofile(os.path.join(d, "in.bin"))
-        O.run_ref_driver(workers=workers, op="reduce_u64", gen="file", out=os.path.join(d, "o.bin"),
-                         **{"in": os.path.join(d, "in.bin")})
-        ref = np.sort(np.fromfile(os.path.join(d, "o.bin"), dtype=REDUCE_OUT), order="key")
+    kv = live_reduce_zero_key_input(workers)
+    n = len(kv)
+    ref = golden_live()["reduce_u64_zero_key_w%d" % workers]
     out, oc = O.reduce_operator(kv, _counts(n, workers), 64 << 20, O.OP_SUM_U64)
     owner = np.repeat(np.arange(workers, dtype=np.uint64), oc.astype(np.int64))
     order = np.argsort(out["key"], kind="stable")
@@ -151,16 +131,11 @@ def test_golden_reduce_to_index_dense_result():
     assert np.count_nonzero((ref["key"] == 0) & (ref["val"] == 0)) > 40000        # mostly neutral
 
 
-@needs_ref
-@pytest.mark.ref
-@pytest.mark.parametrize("workers,n,universe", [(1, 5000, 300), (2, 40000, 7001), (5, 3000, 100000)])
+@pytest.mark.parametrize("workers,n,universe", LIVE_REDUCE_TO_INDEX_CASES)
 def test_live_reference_reduce_to_index(workers, n, universe):
-    """live run of the unmodified reference's ReduceToIndex on a fresh shape (dense, sparse, more workers than data per
-    index): the oracle's dense array is bit-identical in exact mode"""
-    with tempfile.TemporaryDirectory() as d:
-        out = os.path.join(d, "o.bin")
-        O.run_ref_driver(workers=workers, op="reduce_to_index", gen="uniform", universe=universe, n=n, exact=1, out=out)
-        ref = np.fromfile(out, dtype=O.KV)
+    """the unmodified reference's ReduceToIndex on a fresh shape (dense, sparse, more workers than data per index): the
+    oracle's dense array is bit-identical in exact mode"""
+    ref = golden_live()["reduce_to_index_uniform_u%d_%d_exact1_w%d" % (universe, n, workers)]
     assert len(ref) == universe
     mine = O.reduce_to_index(_rti_input("uniform", n, universe, 1), universe, O.OP_SUM_F64)
     assert np.array_equal(mine, ref)
@@ -201,10 +176,10 @@ def test_cfg1_word_count_plumbing_two_loopback_workers(tmp_path):
     assert "words=150000" in line and "workers=2" in res.stdout
     counts = dict((w, int(c)) for w, c in (l.split() for l in open(out)))
     assert sum(counts.values()) == 150000 and 900 <= len(counts) <= 1000
-    sample = "/root/reference/tests/inputs/wordcount.in"
-    if os.path.exists(sample):           # the reference's own fixture (tests/examples/word_count_test.cpp: 71 pairs), in this container only
-        res = subprocess.run([O.REF_DRIVER, "op=word_count", "gen=file", "in=" + sample, "out=" + out], env=env, capture_output=True, text=True, timeout=600)
-        assert res.returncode == 0
-        got = dict((w, int(c)) for w, c in (l.split() for l in open(out)))
-        want = collections.Counter(open(sample).read().split())
-        assert got == dict(want) and len(got) == 71
+    # the reference's own fixture (its tests/inputs/wordcount.in, checked by tests/examples/word_count_test.cpp: 71 pairs)
+    sample = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "wordcount.in")
+    res = subprocess.run([O.REF_DRIVER, "op=word_count", "gen=file", "in=" + sample, "out=" + out], env=env, capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0
+    got = dict((w, int(c)) for w, c in (l.split() for l in open(out)))
+    want = collections.Counter(open(sample).read().split())
+    assert got == dict(want) and len(got) == 71
